@@ -34,6 +34,19 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
 
 ALGO_BYTES_VERIFY = 128.125   # SURVEY §8(d): 64 B sig + 32 B pk + 32 B digest in, 1 bit out
 ALGO_BYTES_DIGEST = 512 + 32  # bytes hashed + digest out
+DUMP_MAX_ELEMS = 1 << 22      # per array written by --dump-outputs: 16 MB of float32
+
+
+def write_outputs(out_dir, **arrays):
+    """--dump-outputs: writes each array as out_dir/<name>.npy in float32.  An array of more than DUMP_MAX_ELEMS elements is cut
+    down to a fixed sample of its rows (seed 0, in row order), the same in every run with the same arguments, so that two builds
+    of the project can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        rows = max(1, DUMP_MAX_ELEMS // max(1, int(np.prod(a.shape[1:]))))
+        if a.shape[0] > rows:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], rows, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------ input synthesis
@@ -381,7 +394,14 @@ def main():
     ap.add_argument("--committee", type=int, default=1000)
     ap.add_argument("--qcs", type=int, default=10000)
     ap.add_argument("--votes-per-qc", type=int, default=100)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float32): accept.npy = the 0/1 verdict "
+                         "of every record of every rank, digest.npy = rank 0's 32-byte digests (a fixed sample of rows above 2^22 values)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "msgs"):
+        ap.error("--dump-outputs applies to the GPU arm's msgs workload")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -487,6 +507,11 @@ def main():
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
+    if args.dump_outputs and rank == 0:
+        # taken before the kernel timings below overwrite d_bitmap and d_digest
+        words_all = (pag.full if pag is not None else d_all) if world > 1 else d_bitmap
+        accept = np.unpackbits(words_all.cpu().numpy().view(np.uint8).reshape(world, -1), axis=1, bitorder="little")[:, :n].reshape(-1)
+        write_outputs(args.dump_outputs, accept=accept, digest=d_digest.cpu().numpy())
     total_ms = ev[0].elapsed_time(ev[-1])
     launches = eng.kernel_launches - launches0
     # dominant kernel timed on its own (same stream, CUDA events around the verify pass only: digests already computed)
@@ -552,14 +577,15 @@ def main():
     if world > 1:
         dist.barrier()
     launches_e2e0 = eng.kernel_launches
+    e2e_steps = 1 if args.no_e2e else args.steps
     t0 = time.perf_counter()
-    for _ in range(1 if args.no_e2e else args.steps):
+    for _ in range(e2e_steps):
         step_e2e()
     dt = time.perf_counter() - t0
     t = torch.tensor([dt], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    e2e = {"value": world * n * args.steps / float(t.item()), "unit": "verifies/s", "h2d_bytes_per_step": int(h_bytes), "d2h_bytes_per_step": int(words * 4),
+    e2e = {"value": world * n * e2e_steps / float(t.item()), "unit": "verifies/s", "h2d_bytes_per_step": int(h_bytes), "d2h_bytes_per_step": int(words * 4),
            "api": "hs_verify_msgs (host pointers, pinned)", "gpu_launches": int(eng.kernel_launches - launches_e2e0)}
     clocks = sampler.stop() if rank == 0 else None
 
@@ -580,7 +606,7 @@ def main():
     # total, sharded across the ranks, every rank ends with every verdict).  Re-registers the committee (untimed, epoch set-up).
     strong = None
     if not args.no_strong:
-        strong = qc_leg(eng, torch, dist, dev, rank, world, 10000, 150, 6667, max(5, args.steps), args.warmup, args.collective)
+        strong = qc_leg(eng, torch, dist, dev, rank, world, 10000, 150, 6667, args.steps, args.warmup, args.collective)
     if rank == 0:
         peaks = {}
         try:
